@@ -2,7 +2,7 @@
 """Benchmark of the Feature2Face generator hot path (BASELINE.json: 512x512 frames/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--mode parity|fast] [--variant large|normal]
-                    [--height H --width W] [--gather auto|ce|nccl] [--clip-frames F] [--impl reference]
+                    [--height H --width W] [--gather auto|ce|nccl] [--clip-frames F] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the generator over one batch of B synthetic frames (default: the May.yaml 'large' network at
 512x512, 32 frames per step - BASELINE.json configs[1]; frames of a clip are independent, so the clip is rendered B
@@ -13,6 +13,7 @@ Prints ONE JSON line on rank 0.  See DESIGN.md "Measurement" for every field.
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -31,6 +32,7 @@ import torch  # noqa: E402
 
 RECIPE = "A"
 CLIP_FRAMES = 672          # frames demo.py renders for data/Input/00083.wav (SURVEY.md 8d): the end-to-end clip
+DUMP_LIMIT = 64_000_000 - 4096     # bytes of array data --dump-outputs may write: 64 MB less room for the .npy header
 
 
 def parse():
@@ -53,6 +55,9 @@ def parse():
                     help="N > 1: also render one clip of exactly this many frames and report it as clip_run (BASELINE.json "
                          "configs[3]: 10000 synthetic frames, frame-sharded; 0 = skip)")
     ap.add_argument("--no-extras", action="store_true", help="skip the side measurements (other modes / configs, library baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the fp32 frames of the last timed step to DIR/frames.npy (a fixed sample "
+                         "of them when they exceed 64 MB), so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -111,6 +116,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100",
                                           "-i", str(self.gpu)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)            # no sampler outlives a run that fails before stop()
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -149,6 +155,27 @@ def make_net(variant: str, mode: str):
     sd = O.make_state_dict(variant, RECIPE)
     net.load_state_dict(sd, strict=True)
     return net.cuda().eval(), sd
+
+
+def dump_outputs(dirpath: str, frames: torch.Tensor) -> None:
+    """DIR/frames.npy: the fp32 frames ``[n, 3, H, W]`` of the last timed step, all of them when they fit in DUMP_LIMIT bytes;
+    else the frames at fixed seeded indices, or, when one frame alone is larger, every k-th element of the flattened frames."""
+    x = frames.detach().float()
+    note = "all frames"
+    if x.numel() * 4 > DUMP_LIMIT:
+        per_frame = x[0].numel() * 4
+        if per_frame <= DUMP_LIMIT:
+            idx = np.sort(np.random.default_rng(0).choice(x.shape[0], DUMP_LIMIT // per_frame, replace=False))
+            x = x[torch.from_numpy(idx).to(x.device)]
+            note = f"frames {idx.tolist()}"
+        else:
+            k = -(-x.numel() // (DUMP_LIMIT // 4))
+            x = x.reshape(-1)[::k]
+            note = f"every {k}-th element"
+    os.makedirs(dirpath, exist_ok=True)
+    path = os.path.join(dirpath, "frames.npy")
+    np.save(path, x.cpu().numpy())
+    print(f"bench: wrote {path} {tuple(x.shape)} float32 ({note} of the last timed step, {tuple(frames.shape)})", file=sys.stderr)
 
 
 _CPU_THREADS = None
@@ -374,6 +401,8 @@ def main():
         checks = sorted({0, B // 2, B - 1})
         parity_err = max(oracle_err(last[j:j + 1], 0, K - 1, j) for j in checks)
         parity_note = f"frames {checks} of the last timed {B}-frame step vs the oracle"
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
     else:
         # N > 1: the library's own multi-GPU entry point.  One render() = K chunks of B frames per rank; the tail kernel writes
         # into the clip buffer, the frames travel to every rank (copy engines over symmetric memory, or NCCL all-gather).
@@ -407,6 +436,10 @@ def main():
                 errs.append(oracle_err(clip_all[g:g + 1], r, st_, j))
             parity_err = max(errs)
             parity_note = f"frames (rank, step, index) {picks} of the gathered clip on rank 0 vs the oracle"
+            if args.dump_outputs:
+                # the last timed step of every rank: frames (K-1)*B ... K*B-1 of each rank's block of the gathered clip
+                starts = [partition(K * B * world, world, r)[0] + (K - 1) * B for r in range(world)]
+                dump_outputs(args.dump_outputs, torch.cat([clip_all[s0:s0 + B] for s0 in starts]))
     ms_total = e0.elapsed_time(e1)
     ms_step_local = ms_total / K
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None

@@ -95,8 +95,6 @@ struct alignas(64) ConvParams {
   int32_t tiles_x, tiles_y, tiles_n;
   int32_t n_phases;
   int32_t trace_skip;        // debug: the trace records local tiles [trace_skip, trace_skip + kTraceTiles)
-  int32_t debug_fault;       // test hook (LSPG_DEBUG_FAULT_LAYER): the producer withholds one activation tile, so a barrier never
-                             // completes and the bounded mbar_wait traps - the error path of a pipeline bug, on purpose
   FastDiv fd_tps, fd_m_tiles, fd_n_tiles, fd_tiles_x, fd_tiles_y;   // divisions of decode_tile (tiles_per_split, ...)
   // ---- MMA issue + TMA producer
   uint32_t idesc;            // UMMA instruction descriptor (M=128 or 256, N=BN, bf16 x bf16 -> f32, K-major)
@@ -705,8 +703,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
           if (!early) ptx::mbar_expect_tx(&full_bar[stage], Cfg::kStage);
 #pragma unroll
           for (int l = 0; l < NL; ++l) {
-            if (!(p.debug_fault && issued == 0 && l == 0))
-              ptx::tma_load_5d(&p.a[amap + s], &full_bar[stage], st + l * kATile, c * kChunk, xx, yy, tc.n0, l);
+            ptx::tma_load_5d(&p.a[amap + s], &full_bar[stage], st + l * kATile, c * kChunk, xx, yy, tc.n0, l);
             if (!early)
               ptx::tma_load_3d(&p.w, &full_bar[stage], st + NL * kATile + l * Cfg::kBTile, kb * kChunk, tc.nt * BN,
                                l * p.n_phases + tc.z);

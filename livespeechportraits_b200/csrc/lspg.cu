@@ -820,10 +820,6 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
         p.trace_skip = ts ? atoi(ts) : 0;
       }
     }
-    {
-      const char* fl = getenv("LSPG_DEBUG_FAULT_LAYER");      // test hook: see ConvParams::debug_fault
-      if (fl && atoi(fl) == static_cast<int>(P->layers.size()) && !g.patch) p.debug_fault = 1;
-    }
     if (pl.split) {
       ReduceParams& r = pl.red;
       memset(&r, 0, sizeof(r));

@@ -19,6 +19,7 @@ from oracle import a2h_oracle as A  # noqa: E402
 
 
 def main():
+    torch.set_num_threads(8)          # tests/test_a2h_oracle.py GOLDEN_THREADS: the loop's last bits depend on it
     opt = A.default_opt()
     recipe, wseed, aseed, tseed, n_audio, sigma = "B", 0, 1, 5, 60, 0.3
     sd = A.make_state_dict(opt, recipe, wseed)

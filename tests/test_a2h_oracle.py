@@ -1,5 +1,5 @@
-"""Row N4 (SURVEY.md 8f), CPU part: the oracle of the Audio2Headpose loop pinned against the live reference and against
-golden vectors generated from it; the incremental recurrence the CUDA kernel runs checked against the oracle - in its
+"""Row N4 (SURVEY.md 8f), CPU part: the oracle of the Audio2Headpose loop pinned against golden vectors generated from the
+reference; the incremental recurrence the CUDA kernel runs checked against the oracle - in its
 float64 host emulator (algorithmic equivalence) and with the arrays lsph_load_weights actually packed (host logic of the
 C ABI, no GPU); the C ABI's argument checking."""
 import ctypes as C
@@ -16,6 +16,19 @@ import a2h_incremental as INC
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "a2h_B_60.npz")
+GOLD_LOOP = os.path.join(os.path.dirname(__file__), "golden", "a2h_live_loop.npz")
+# Intra-op CPU threads the reference ran with when tests/golden/a2h_*.npz were written.  ATen's CPU matmuls split their
+# sums by thread count (1 or 12+ threads round differently from 2-8), and the loop feeds those last bits back into its
+# history, so the restatement reproduces the stored vectors only with the same count.
+GOLDEN_THREADS = 8
+
+
+@pytest.fixture
+def golden_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def test_known_answers():
@@ -28,6 +41,7 @@ def test_known_answers():
     assert sum(int(np.prod(s)) for k, s in spec.items() if not k.endswith("num_batches_tracked")) == 4267939
 
 
+@pytest.mark.usefixtures("golden_threads")
 def test_oracle_matches_golden_from_the_reference():
     """tests/golden/a2h_B_60.npz was written by oracle/make_golden_a2h.py from the UNMODIFIED Audio2HeadposeModel."""
     g = np.load(GOLD)
@@ -41,30 +55,26 @@ def test_oracle_matches_golden_from_the_reference():
     assert np.abs(params - g["params"]).max() <= 2e-6
 
 
-@pytest.mark.skipif(not A.reference_available(), reason="reference checkout not present on this machine")
+@pytest.mark.usefixtures("golden_threads")
 def test_oracle_matches_the_live_reference_loop():
+    """tests/golden/a2h_live_loop.npz holds what the UNMODIFIED Audio2HeadposeModel computed (oracle/make_golden_reference_checks.py):
+    its key list, its generate_sequences loop under torch.manual_seed(11) and one full-window forward of its module."""
+    g = np.load(GOLD_LOOP)
     opt = A.default_opt()
+    assert list(g["keys"]) == list(A.state_dict_spec(opt).keys())
     for recipe, seed in (("A", 1), ("B", 2)):
         sd = A.make_state_dict(opt, recipe, seed)
-        m = A.reference_model(opt, sd)
-        net = m.Audio2Headpose
-        assert list(net.state_dict().keys()) == list(A.state_dict_spec(opt).keys())
         audio = A.make_audio_feats(36, opt, seed)
         pre = np.linspace(-0.2, 0.3, 12).astype(np.float32)
         noise = A.reference_noise(36 - 15, 12, 1, seed=11)
-        torch.manual_seed(11)
-        import contextlib
-        import io
-        with contextlib.redirect_stderr(io.StringIO()):
-            ref = m.generate_sequences(audio.copy(), pre, fill_zero=True, sigma_scale=0.3, opt=opt)
         mine = A.generate_sequences(sd, audio, pre, noise, opt, 0.3)
+        ref = g[f"{recipe}_pred"]
         assert ref.shape == (21, 12) and ref.dtype == np.float64
         assert np.abs(ref - mine).max() <= 1e-6, recipe
         # one full-window forward against the module's own forward
-        hist = torch.randn(1, 255, 12)
+        hist = torch.from_numpy(np.random.Generator(np.random.PCG64(11)).standard_normal((1, 255, 12)).astype(np.float32))
         aud = torch.from_numpy(A.make_audio_feats(255, opt, 5)).unsqueeze(0)
-        with torch.no_grad():
-            assert torch.allclose(net(hist, aud), A.audio2headpose_forward(sd, hist, aud, opt), atol=1e-6)
+        assert torch.allclose(torch.from_numpy(g[f"{recipe}_forward"]), A.audio2headpose_forward(sd, hist, aud, opt), atol=1e-6)
 
 
 @pytest.mark.parametrize("recipe", ["A", "B"])

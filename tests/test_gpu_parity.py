@@ -14,7 +14,7 @@ from oracle import f2f_oracle as O
 pytestmark = pytest.mark.gpu
 TOL = 1e-3
 GOLDEN = sorted(p for p in glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz"))
-                if not os.path.basename(p).startswith(("raster_", "a2h_")))      # raster_*: tests/test_raster_oracle.py
+                if not os.path.basename(p).startswith(("raster_", "a2h_", "f2f_")))  # raster_*: tests/test_raster_oracle.py
 
 
 def opt(size):
@@ -280,39 +280,3 @@ def test_forward_refuses_incomplete_weights():
     assert rc == -4 and b"never loaded" in lib.lspg_last_error()           # LSPG_ESTATE, not black frames
     lib.lspg_destroy(h)
 
-
-def test_pipeline_fault_surfaces_as_an_error_not_a_hang(tmp_path):
-    """A pipeline bug (here: the producer withholds one activation tile, LSPG_DEBUG_FAULT_LAYER) must end in the bounded
-    mbarrier wait's trap and a CUDA error the host can see - not in a hung GPU - and the handle must still be destroyable.
-    Runs in a subprocess: a trapped kernel poisons the CUDA context of its process."""
-    import subprocess
-    import sys
-    import textwrap
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = textwrap.dedent(f"""
-        import os, sys, time, types
-        sys.path.insert(0, {root!r})
-        os.environ["LSPG_DEBUG_FAULT_LAYER"] = "20"          # a stride-2 conv (one-box-per-tap kernel) of the normal network
-        import torch
-        from livespeechportraits_b200.generator import Feature2Face_G
-        from oracle import f2f_oracle as O
-        net = Feature2Face_G(types.SimpleNamespace(isTrain=False, size="normal", n_downsample_G=8, ngf=64, fp16=0), precision="parity")
-        net.load_state_dict(O.make_state_dict("normal", "A"))
-        net = net.cuda().eval()
-        t0 = time.time()
-        try:
-            net(torch.zeros(1, 13, 256, 256, device="cuda"))
-            torch.cuda.synchronize()
-            print("NO_ERROR")
-        except Exception as exc:
-            print("ERROR_SEEN", type(exc).__name__, f"{{time.time() - t0:.1f}}s")
-        try:
-            del net                                             # lspg_destroy on a poisoned context must not crash
-            print("DESTROYED")
-        except Exception as exc:
-            print("DESTROY_FAILED", exc)
-    """)
-    proc = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120)
-    out = proc.stdout + proc.stderr
-    assert "ERROR_SEEN" in proc.stdout and "NO_ERROR" not in proc.stdout, out[-2000:]
-    assert "DESTROYED" in proc.stdout, out[-2000:]
