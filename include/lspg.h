@@ -138,8 +138,15 @@ typedef struct lspg_layer_geo {
   int64_t partial_bytes; /* fp32 split-K partials this layer needs in the scratch region (0 for a cluster split) */
   int cluster_split;     /* > 0: the n_split CTAs of a tile are one thread-block cluster and reduce through distributed shared
                             memory (no finisher launch); then n_split == cluster_split in {2, 4, 8} */
+  int cta_cluster;       /* CTAs per thread-block cluster of the launch: 2 for the pair kernel and for a patch kernel that
+                            multicasts its weights, cluster_split for a cluster split, 1 otherwise */
 } lspg_layer_geo;
 int lspg_debug_layer_geo(lspg_handle h, int layer, int batch, int height, int width, lspg_layer_geo* out);
+
+/* Byte offset of limb `limb` of activation tensor `id` in the workspace of a (batch,height,width,mode) forward, counted from
+ * the first 1024-byte-aligned address of the workspace (where the launch plan places tensor 0).  Host logic only; works on
+ * a host-only handle.  Lets a caller view the stored activations in place. */
+int lspg_debug_tensor_offset(lspg_handle h, int id, int limb, int batch, int height, int width, int mode, size_t* offset);
 
 /* Test hook (host only, no device): q = n / d computed exactly as the kernels' tile decode does it (multiply-high by a
  * launch-time constant, csrc/conv_umma.cuh make_fast_div / fast_div); valid for n < 2^31, d >= 1. */

@@ -16,7 +16,7 @@ SYMBOLS = [
     "lspg_num_layers", "lspg_layer_info_get", "lspg_layer_packed", "lspg_layer_affine", "lspg_num_tensors",
     "lspg_tensor_shape", "lspg_debug_read_tensor", "lspg_launches_per_forward", "lspg_flops_per_frame",
     "lspg_profile_enable", "lspg_profile_read", "lspg_debug_read_trace", "lspg_debug_fast_div", "lspg_debug_layer_geo",
-    "lspg_graph_stats", "lspg_release_workspace",
+    "lspg_graph_stats", "lspg_release_workspace", "lspg_debug_tensor_offset",
 ]
 
 # include/lsph.h (Audio2Headpose generation loop)
@@ -46,7 +46,8 @@ class LspgLayerInfo(C.Structure):
 class LspgLayerGeo(C.Structure):
     _fields_ = [("kernel", C.c_int), ("bn", C.c_int), ("tile_w", C.c_int), ("tile_h", C.c_int), ("tile_n", C.c_int),
                 ("m_tiles", C.c_int), ("n_tiles", C.c_int), ("n_phases", C.c_int), ("n_split", C.c_int), ("split_len", C.c_int),
-                ("k_items", C.c_int), ("ctas", C.c_int), ("partial_bytes", C.c_int64), ("cluster_split", C.c_int)]
+                ("k_items", C.c_int), ("ctas", C.c_int), ("partial_bytes", C.c_int64), ("cluster_split", C.c_int),
+                ("cta_cluster", C.c_int)]
 
 
 class LspgError(RuntimeError):
@@ -91,6 +92,8 @@ def load(build_if_missing: bool = True) -> C.CDLL:
                                  C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
     lib.lspg_forward_image.argtypes = lib.lspg_forward.argtypes
     lib.lspg_debug_layer_geo.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(LspgLayerGeo)]
+    lib.lspg_debug_tensor_offset.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                             C.POINTER(C.c_size_t)]
     lib.lspg_debug_fast_div.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32)]
     lib.lspg_draw_feature_maps.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                            C.c_void_p]

@@ -475,6 +475,7 @@ struct Geo {
   size_t partial_bytes;
   bool pair;                   // conv_pair_kernel: cta_group::2 UMMA over a 2-CTA cluster (wide layers)
   int csplit;                  // > 0: split-K inside a thread-block cluster of this many CTAs (DSMEM reduction, no finisher)
+  int cluster;                 // CTAs per cluster of the launch: 2 = pair / weight multicast, csplit, else 1
 };
 
 Geo layer_geo(const lspg_ctx* h, const Layer& L, int B, int H, int W) {
@@ -557,6 +558,12 @@ Geo layer_geo(const lspg_ctx* h, const Layer& L, int B, int H, int W) {
       else g.split_len = g.k_items;
     }
   }
+  // A patch-kernel layer that fills at least one wave without split-K runs its CTAs in pairs that share each weight stage
+  // by TMA multicast.
+  static const bool no_cluster = getenv("LSPG_NO_CLUSTER") != nullptr;
+  if (g.pair) g.cluster = 2;
+  else if (g.csplit) g.cluster = g.csplit;
+  else g.cluster = (g.patch && !no_cluster && g.n_split == 1 && g.m_tiles % 2 == 0 && g.tiles_per_split >= sms) ? 2 : 1;
   return g;
 }
 
@@ -570,6 +577,19 @@ size_t workspace_bytes(const lspg_ctx* h, int B, int H, int W, int mode) {
   size_t total = 0;
   for (const auto& t : h->tensors) total += align_up(tensor_bytes_one_limb(t, B, H, W), 1024) * nl_of(mode);
   return total + scratch_bytes(h, B, H, W) + 1024;
+}
+
+// Activation layout inside the workspace, from its first 1024-aligned byte: every tensor's limbs back to back, each limb
+// padded to 1 KB.  Returns the end of the last tensor (where the split-K scratch begins).
+size_t tensor_layout(const lspg_ctx* h, int B, int H, int W, int NL, std::vector<size_t>* off, std::vector<size_t>* limb_stride) {
+  size_t o = 0;
+  for (const auto& t : h->tensors) {
+    const size_t one = align_up(tensor_bytes_one_limb(t, B, H, W), 1024);
+    off->push_back(o);
+    limb_stride->push_back(one);
+    o += one * NL;
+  }
+  return o;
 }
 
 int check_shape(const lspg_ctx* h, int B, int H, int W, int mode) {
@@ -677,15 +697,9 @@ uint32_t make_idesc(int bn, int m, bool f16) {
 int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* workspace) {
   const int NL = nl_of(mode);
   P->batch = B; P->height = H; P->width = W; P->mode = mode; P->workspace = workspace;
-  size_t off = 0;
   const size_t base = align_up(reinterpret_cast<size_t>(workspace), 1024) - reinterpret_cast<size_t>(workspace);
-  off = base;
-  for (const auto& t : h->tensors) {
-    const size_t one = align_up(tensor_bytes_one_limb(t, B, H, W), 1024);
-    P->tensor_off.push_back(off);
-    P->tensor_limb_stride.push_back(one);
-    off += one * NL;
-  }
+  const size_t off = base + tensor_layout(h, B, H, W, NL, &P->tensor_off, &P->tensor_limb_stride);
+  for (auto& o : P->tensor_off) o += base;
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   uint8_t* ws_scratch = ws + align_up(off, 1024);
   for (const Layer& L : h->layers) {
@@ -773,9 +787,8 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
     const int used = (L.kind == K_S2) ? 4 : L.n_src;
     for (int q = used; q < 4; ++q) p.a[q] = p.a[0];
     if (pl.patch) {
-      static const bool no_cluster = getenv("LSPG_NO_CLUSTER") != nullptr;
       pl.pair = g.pair;
-      pl.cluster = (g.pair || (!no_cluster && g.n_split == 1 && g.m_tiles % 2 == 0 && g.tiles_per_split >= h->num_sms)) ? 2 : 1;
+      pl.cluster = g.csplit ? 1 : g.cluster;     // a cluster split launches CL = 1 code in clusters of csplit CTAs
       if (pl.cluster == 1 && NL == 1 && !pl.pair) rc = make_weight_map_taps(h, &p.w, L, pl.bn, patch_tps(pl.bn, NL, L.kind == K_TAIL), NL);
       else rc = make_weight_map_taps(h, &p.w, L, pl.bn / pl.cluster, 1, NL);      // per-tap boxes (row slice per CTA when multicasting)
       if (rc) return rc;
@@ -1387,6 +1400,19 @@ int lspg_debug_layer_geo(lspg_handle h, int layer, int batch, int height, int wi
   o->ctas = ctas;
   o->partial_bytes = static_cast<int64_t>(g.partial_bytes);
   o->cluster_split = g.csplit;
+  o->cta_cluster = g.cluster;
+  return LSPG_OK;
+}
+
+int lspg_debug_tensor_offset(lspg_handle h, int id, int limb, int batch, int height, int width, int mode, size_t* offset) {
+  if (!h || !offset) return fail(LSPG_EINVAL, "null argument");
+  int rc = check_shape(h, batch, height, width, mode);
+  if (rc) return rc;
+  if (id < 0 || id >= static_cast<int>(h->tensors.size())) return fail(LSPG_EINVAL, "tensor %d out of range", id);
+  if (limb < 0 || limb >= nl_of(mode)) return fail(LSPG_EINVAL, "limb %d not present in this mode", limb);
+  std::vector<size_t> off, limb_stride;
+  tensor_layout(h, batch, height, width, nl_of(mode), &off, &limb_stride);
+  *offset = off[id] + static_cast<size_t>(limb) * limb_stride[id];
   return LSPG_OK;
 }
 

@@ -245,6 +245,16 @@ def test_planner_invariants(variant, batch):
                 assert g.partial_bytes == g.n_split * tiles * 128 * g.bn * 4
         else:
             assert g.partial_bytes == 0 and g.cluster_split == 0
+        # the launch's cluster: CTA pairs, the CTAs of a cluster split, or pairs of patch CTAs that multicast their weight
+        # stages when the layer fills a wave without split-K
+        if g.kernel == 2:
+            assert g.cta_cluster == 2
+        elif g.cluster_split:
+            assert g.cta_cluster == g.cluster_split
+        elif g.kernel == 1:
+            assert g.cta_cluster == (2 if g.n_split == 1 and g.m_tiles % 2 == 0 and tiles >= sms else 1)
+        else:
+            assert g.cta_cluster == 1
         assert 1 <= g.ctas <= sms
     assert ws > max(g.partial_bytes for _, g in table)
     n_split_layers = sum(1 for _, g in table if g.n_split > 1)
@@ -253,6 +263,49 @@ def test_planner_invariants(variant, batch):
         assert n_split_layers >= 10 and n_cluster == n_split_layers       # from 8 frames up every split layer reduces inside its cluster
     else:
         assert n_cluster == 0 and (batch != 1 or n_split_layers >= 40)     # below that (measured slower) the finisher kernel stays
+
+
+@pytest.mark.parametrize("variant,batch,height,width,mode", [("normal", 1, 256, 256, 1), ("normal", 3, 512, 256, 0),
+                                                             ("large", 32, 512, 512, 1), ("large", 5, 256, 1024, 0)])
+def test_tensor_offsets_are_aligned_disjoint_and_inside_the_workspace(variant, batch, height, width, mode):
+    """lspg_debug_tensor_offset: every limb of every activation tensor starts on a 1 KB boundary of the aligned workspace,
+    no two overlap, and all of them - and the split-K scratch after them - fit in lspg_workspace_bytes minus the slack that
+    aligning the caller's pointer may use."""
+    lib = _lib.load()
+    h = C.c_void_p()
+    assert lib.lspg_create(C.byref(h), _lib.LSPG_VARIANT[variant], 64, 8, 13, 3, -1) == 0
+    try:
+        need = C.c_size_t()
+        assert lib.lspg_workspace_bytes(h, batch, height, width, mode, C.byref(need)) == 0
+        nt = C.c_int()
+        lib.lspg_num_tensors(h, C.byref(nt))
+        spans = []
+        for t in range(nt.value):
+            c, th, tw = C.c_int(), C.c_int(), C.c_int()
+            assert lib.lspg_tensor_shape(h, t, height, width, C.byref(c), C.byref(th), C.byref(tw)) == 0
+            nbytes = batch * th.value * tw.value * c.value * 2
+            for limb in range(2 if mode == 1 else 1):
+                off = C.c_size_t()
+                assert lib.lspg_debug_tensor_offset(h, t, limb, batch, height, width, mode, C.byref(off)) == 0
+                assert off.value % 1024 == 0
+                spans.append((off.value, off.value + nbytes))
+        spans.sort()
+        assert spans[0][0] == 0
+        assert all(a[1] <= b[0] for a, b in zip(spans, spans[1:])), "activation tensors overlap"
+        n = C.c_int()
+        lib.lspg_num_layers(h, C.byref(n))
+        partial = 0
+        for i in range(n.value):
+            g = _lib.LspgLayerGeo()
+            assert lib.lspg_debug_layer_geo(h, i, batch, height, width, C.byref(g)) == 0
+            partial = max(partial, g.partial_bytes)
+        assert -(-spans[-1][1] // 1024) * 1024 + partial <= need.value - 1024
+        off = C.c_size_t()
+        assert lib.lspg_debug_tensor_offset(h, nt.value, 0, batch, height, width, mode, C.byref(off)) == -1
+        assert lib.lspg_debug_tensor_offset(h, 0, 2 if mode == 1 else 1, batch, height, width, mode, C.byref(off)) == -1
+        assert lib.lspg_debug_tensor_offset(h, 0, 0, batch, 300, width, mode, C.byref(off)) == -1
+    finally:
+        lib.lspg_destroy(h)
 
 
 def test_planner_picks_the_n_tile_with_fewer_waves():
