@@ -37,8 +37,6 @@ constexpr int kChunk = 64;                  // channels per K block = 128 bytes 
 constexpr int kATile = kTileM * 128;        // bytes of one A (or staging) tile
 constexpr int kMaxTaps = 9;
 constexpr int kThreads = 192;            // 2 role warps + 4 epilogue warps
-constexpr int kThreadsWide = 320;        // 2 role warps + 8 epilogue warps (patch / pair kernels, non-tail)
-constexpr int kEpiThreads = 128;
 constexpr int kSmemBudget = 227 * 1024;
 
 // Division by a launch-time constant as multiply-high + shift (dividend < 2^31): decode_tile runs between two tiles of
@@ -87,7 +85,7 @@ struct alignas(64) ConvParams {
   int32_t total_tiles;       // tiles_x*tiles_y*tiles_n * n_tiles * n_phases * n_split
   // split-K: the K loop (v1: K blocks; patch mode: (source, chunk) items) is cut into n_split ranges of split_len;
   // tile index = split * tiles_per_split + tile.  Each CTA writes its raw fp32 accumulator tile to
-  // partial[tile_index][128][BN]; splitk_reduce_kernel sums the splits and applies the epilogue.
+  // partial[tile_index][128][BN]; splitk_reduce_kernel (given these same parameters) sums the splits and finishes the tile.
   int32_t n_split, tiles_per_split;
   int32_t cluster_split;     // 1: the n_split CTAs of a tile form a thread-block cluster and reduce their partials through
                              // distributed shared memory (CSP kernel variants); 0: partials go to `partial` + finisher kernel
@@ -106,7 +104,6 @@ struct alignas(64) ConvParams {
   // patch mode: one halo patch {64 ch, patch_w, patch_h} per (tile, source, chunk) whose origin is the tile origin +
   // (patch_dx0, patch_dy0)[phase]; every tap is a row offset inside the patch.
   int32_t patch_w, patch_h;
-  int32_t desc_base_offset;      // 1: set the UMMA descriptor base-offset field from the start address (bring-up switch)
   int8_t patch_dx0[4], patch_dy0[4];
   int16_t tap_row[4][kMaxTaps];  // [phase][tap] -> first patch row of the tap's shifted A tile
   int8_t tap_map[4][kMaxTaps];   // [phase][tap] -> index into a[] (added to the concat source index)
@@ -115,7 +112,6 @@ struct alignas(64) ConvParams {
   // ---- tensor maps
   CUtensorMap a[4];          // activation views: [parity or concat source], dims {C, X, Y, N, limb}
   CUtensorMap w;             // packed weights, dims {K, Cout_pad, limb*n_phases + phase}
-  CUtensorMap out[4];        // output views per phase, dims {C, X, Y, N, limb}
 };
 
 // CSP ("cluster split"): split-K inside a thread-block cluster.  The n_split (2, 4 or 8) CTAs that share an output tile are
@@ -126,7 +122,6 @@ template <int BN, int NL, bool TAIL, bool CSP = false>
 struct ConvCfg {
   static constexpr int kBTile = BN * 128;
   static constexpr int kStage = NL * (kATile + kBTile);
-  static constexpr int kNumStg = 0;                                  // (no smem staging of results: the epilogue writes global memory directly)
   static constexpr int kStgBytes = CSP ? kTileM * BN * 4 : 0;        // cluster split-K: partial rows from the cluster's CTAs
   static constexpr int kAux = 3072;                                  // 2 x (scale, shift) + barriers + tmem ptr
   static constexpr int kAvail = kSmemBudget - 1024 /*alignment slack*/ - kStgBytes - kAux;
@@ -136,7 +131,8 @@ struct ConvCfg {
   static constexpr int kTmemCols = (2 * BN < 32) ? 32 : 2 * BN;
   static_assert(kStages >= 2, "pipeline needs at least two stages");
   static_assert(BN % 16 == 0 && BN >= 16 && BN <= 256, "invalid UMMA N");
-  static_assert(4 * BN * 4 + 256 <= kAux, "aux region too small");
+  // scale/shift, full/empty per stage, tfull/tempty per accumulator buffer, TMEM address
+  static_assert(4 * BN * 4 + (2 * kStages + 2 * 2 + 1) * 8 <= kAux, "aux region too small");
 };
 
 // Debug trace layout per CTA: [0] kernel entry, [1] prologue done, then per local tile i (up to kTraceTiles):
@@ -231,24 +227,94 @@ __device__ __forceinline__ float unpack_hi(uint32_t u) {
   else return bf16_hi(u);
 }
 
-
-template <int NSTG>
-struct StgCfg {
-  static constexpr int kNumStg = NSTG;
+// Output pixel of row `row` of tile `tc`: image n and sampling-grid position (y, x), whether it lies inside the image, and the
+// element offset of its channel 0 in the NHWC output (limb 0).  A folded x2 upsample stores phase z at (2y + z/2, 2x + z%2).
+struct OutPixel {
+  int n, y, x;
+  bool ok;
+  size_t out;
 };
+__device__ __forceinline__ OutPixel out_pixel(const ConvParams& p, const TileCoord& tc, int row) {
+  OutPixel o;
+  o.n = tc.n0 + (row >> (p.tw_log2 + p.th_log2));
+  o.y = tc.y0 + ((row >> p.tw_log2) & ((1 << p.th_log2) - 1));
+  o.x = tc.x0 + (row & ((1 << p.tw_log2) - 1));
+  o.ok = o.n < p.batch && o.y < p.hs && o.x < p.ws;
+  const int oh = p.out_up ? 2 * p.hs : p.hs, ow = p.out_up ? 2 * p.ws : p.ws;
+  const int oy = p.out_up ? 2 * o.y + (tc.z >> 1) : o.y, ox = p.out_up ? 2 * o.x + (tc.z & 1) : o.x;
+  o.out = ((static_cast<size_t>(o.n) * oh + oy) * ow + ox) * p.out_channels;
+  return o;
+}
+// the residual has the output's sampling grid (residual layers are never upsampling ones)
+__device__ __forceinline__ size_t res_offset(const ConvParams& p, const OutPixel& o) {
+  return ((static_cast<size_t>(o.n) * p.hs + o.y) * p.ws + o.x) * p.res_channels;
+}
 
-// Epilogue role (warps 2..5, 128 threads): drains the TMEM accumulators of every tile this CTA owns.
-// NSTG = number of residual-in / result-out staging buffers behind `stg_base`.
+// The last steps of every conv output, shared by the epilogue and both split-K finishers so that they round alike.  y holds
+// C channels of one pixel that already went through the folded BatchNorm (fmaf(acc, scale, shift)); res[l] holds the C / 2
+// packed residual words of limb l (read only with has_res).  Adds the residual limbs in limb order, applies ReLU and rounds to
+// the 16-bit hi limb (hi: C / 2 packed words); for NL == 2 also to the lo limb y - hi.
+template <int NL, int C>
+__device__ __forceinline__ void finish_channels(float (&y)[C], const uint32_t (&res)[NL][C / 2], bool has_res, bool relu,
+                                                uint32_t (&hi)[C / 2], uint32_t (&lo)[C / 2]) {
+  constexpr bool F16 = NL == 2;
+  if (has_res) {
+#pragma unroll
+    for (int l = 0; l < NL; ++l)
+#pragma unroll
+      for (int e = 0; e < C / 2; ++e) {
+        y[2 * e] += unpack_lo<F16>(res[l][e]);
+        y[2 * e + 1] += unpack_hi<F16>(res[l][e]);
+      }
+  }
+  if (relu) {
+#pragma unroll
+    for (int e = 0; e < C; ++e) y[e] = fmaxf(y[e], 0.0f);
+  }
+#pragma unroll
+  for (int e = 0; e < C / 2; ++e) hi[e] = pack2<F16>(y[2 * e], y[2 * e + 1]);
+  if constexpr (F16) {
+#pragma unroll
+    for (int e = 0; e < C / 2; ++e) lo[e] = pack2<true>(y[2 * e] - unpack_lo<true>(hi[e]), y[2 * e + 1] - unpack_hi<true>(hi[e]));
+  }
+}
+
+// Split-K finishers: channels [ch, ch + 4) of pixel o from their summed fp32 accumulator, with scale, shift and residual
+// read from global memory.  One thread = one pixel x 4 channels.
+template <int NL>
+__device__ __forceinline__ void finish4(const ConvParams& p, const OutPixel& o, int ch, float4 acc) {
+  const float4 sc = *reinterpret_cast<const float4*>(p.scale + ch), sh = *reinterpret_cast<const float4*>(p.shift + ch);
+  float y[4] = {fmaf(acc.x, sc.x, sh.x), fmaf(acc.y, sc.y, sh.y), fmaf(acc.z, sc.z, sh.z), fmaf(acc.w, sc.w, sh.w)};
+  uint32_t r[NL][2];
+  if (p.has_res) {
+    const __nv_bfloat16* rr = p.res_ptr + res_offset(p, o) + ch;
+#pragma unroll
+    for (int l = 0; l < NL; ++l) {
+      const uint2 v = *reinterpret_cast<const uint2*>(rr + l * p.res_limb_stride);
+      r[l][0] = v.x; r[l][1] = v.y;
+    }
+  }
+  uint32_t hi[2], lo[2];
+  finish_channels<NL, 4>(y, r, p.has_res, p.relu, hi, lo);
+  __nv_bfloat16* out = p.out_ptr + o.out + ch;
+  *reinterpret_cast<uint2*>(out) = make_uint2(hi[0], hi[1]);
+  if constexpr (NL == 2) *reinterpret_cast<uint2*>(out + p.out_limb_stride) = make_uint2(lo[0], lo[1]);
+}
+
+// Epilogue role (warps 2..2+EW-1): drains the TMEM accumulators of every tile this CTA owns.  Per tile it either
+//   * tail: applies scale/shift and tanh and scatters fp32 NCHW or uint8 HWC,
+//   * split-K: dumps the raw fp32 rows (to the owner CTA's staging buffer under CSP, else to `partial`), or
+//   * regular: applies scale/shift from shared memory and finish_channels, and stores NHWC with 256-bit stores.
 // STACK (parity mode of the patch kernel): the accumulator of a tile is 2*BN columns wide - columns [0,BN) hold
 // A_hi*B_hi + A_lo*B_hi, columns [BN,2BN) hold A_hi*B_lo (one N=2BN MMA over the stacked [B_hi;B_lo] tile) - and the
 // epilogue adds the two halves.
 // EW = number of epilogue warps (4 or 8).  A warp may read TMEM lane quarter (warp % 4); with EW = 8 two warps share a
 // quarter and split the columns in interleaved 32-column pieces, which doubles the loads/stores in flight and the issue
 // slots of the epilogue (the 64-channel layers were epilogue-bound with 4 warps: 6.2k cycles vs 3.5k of MMAs per tile).
-template <int BN, int NL, bool TAIL, int NSTG, bool STACK, bool PAIR = false, int EW = 4, int NACC = 2, bool CSP = false>
-__device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg_base, float* s_scale0, float* /*unused*/,
-                                               uint64_t* tfull_bar, uint64_t* tempty_bar, uint64_t* stg_bar,
-                                               uint32_t tmem_base, int warp, int lane, int t0, int tstep) {
+// stg_base: the cluster split-K staging buffer (CSP only).
+template <int BN, int NL, bool TAIL, bool STACK, bool PAIR = false, int EW = 4, int NACC = 2, bool CSP = false>
+__device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg_base, float* s_scale0, uint64_t* tfull_bar,
+                                               uint64_t* tempty_bar, uint32_t tmem_base, int warp, int lane, int t0, int tstep) {
   static_assert(EW == 4 || EW == 8, "4 or 8 epilogue warps");
   static_assert(!(TAIL && EW != 4), "the tail epilogue uses 4 warps");
   constexpr int kEpi = EW * 32;
@@ -288,22 +354,16 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
     ptx::named_bar_sync(1, kEpi);
     cur_nt = nt;
   };
-  // this thread's pixel inside a tile
-  const int tw_ = row & ((1 << p.tw_log2) - 1);
-  const int th_ = (row >> p.tw_log2) & ((1 << p.th_log2) - 1);
-  const int nb_ = row >> (p.tw_log2 + p.th_log2);
   // Residual of this thread's pixel: 32 channels x NL limbs per 32-column piece, always requested one piece ahead - the
   // first piece of a tile while the previous tile is being finished - so that its L2/HBM latency never sits between the
   // accumulator becoming ready and the TMEM buffer being handed back to the MMA warp.
   const bool use_res = !TAIL && p.has_res && p.n_split == 1;
   uint4 rs[NL][4];
   auto load_res = [&](const TileCoord& c, int c32) {
-    const int n = c.n0 + nb_, y = c.y0 + th_, x = c.x0 + tw_;
-    const bool ok = n < p.batch && y < p.hs && x < p.ws;
+    const OutPixel o = out_pixel(p, c, row);
     // rows outside the image read pixel 0 instead (their result is never stored): no branch around the loads, so the
     // destination registers stay plain in-flight load targets until the math consumes them
-    const size_t pix = ok ? (static_cast<size_t>(n) * p.hs + y) * p.ws + x : 0;
-    const __nv_bfloat16* rr = p.res_ptr + pix * p.res_channels + c.nt * BN + c32 * 32;
+    const __nv_bfloat16* rr = p.res_ptr + (o.ok ? res_offset(p, o) : 0) + c.nt * BN + c32 * 32;
 #pragma unroll
     for (int l = 0; l < NL; ++l)
 #pragma unroll
@@ -326,9 +386,6 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
     constexpr int kAccCols = STACK ? 2 * BN : BN;
     const uint32_t t_acc = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * kAccCols;
 
-    const int pn = tc.n0 + nb_, py_ = tc.y0 + th_, px_ = tc.x0 + tw_;
-    const bool pix_ok = pn < p.batch && py_ < p.hs && px_ < p.ws;
-
     ptx::mbar_wait(&tfull_bar[acc], acc_phase);
     ptx::tc_fence_after();
     if (leader) trace_tile(p, lt, 4);
@@ -346,8 +403,9 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
       }
       ptx::tmem_ld_wait();
       release_tmem();
+      const OutPixel pix = out_pixel(p, tc, row);
       const int oh = 2 * p.hs, ow = 2 * p.ws;
-      if (pix_ok && p.out_u8 != nullptr) {
+      if (pix.ok && p.out_u8 != nullptr) {
         // fused util/util.py:tensor2im (reference lines 33-42): (x + 1) / 2 * 255 in fp32, clip to [0,255], truncate to
         // uint8, CHW -> HWC.  This thread owns output pixels (2y+py, 2x+px): per py, 2 pixels x 3 channels = 6 bytes.
 #pragma unroll
@@ -363,13 +421,13 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
               u = fminf(fmaxf(u, 0.0f), 255.0f);
               b[px * 3 + c] = static_cast<uint8_t>(static_cast<int>(u));
             }
-          uint8_t* dst = p.out_u8 + ((static_cast<size_t>(pn) * oh + (2 * py_ + py)) * ow + 2 * px_) * 3;
+          uint8_t* dst = p.out_u8 + ((static_cast<size_t>(pix.n) * oh + (2 * pix.y + py)) * ow + 2 * pix.x) * 3;
           uint16_t* d16 = reinterpret_cast<uint16_t*>(dst);          // 6-byte aligned: 2x * 3 is even
           d16[0] = static_cast<uint16_t>(b[0] | (b[1] << 8));
           d16[1] = static_cast<uint16_t>(b[2] | (b[3] << 8));
           d16[2] = static_cast<uint16_t>(b[4] | (b[5] << 8));
         }
-      } else if (pix_ok) {
+      } else if (pix.ok) {
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
 #pragma unroll
@@ -377,41 +435,26 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
             float2 o;
             o.x = tanhf(__uint_as_float(v[(py * 2 + 0) * 3 + c]) * s_scale[(py * 2 + 0) * 3 + c] + s_shift[(py * 2 + 0) * 3 + c]);
             o.y = tanhf(__uint_as_float(v[(py * 2 + 1) * 3 + c]) * s_scale[(py * 2 + 1) * 3 + c] + s_shift[(py * 2 + 1) * 3 + c]);
-            float* dst = p.out_f32 + ((static_cast<size_t>(pn) * 3 + c) * oh + (2 * py_ + py)) * ow + 2 * px_;
+            float* dst = p.out_f32 + ((static_cast<size_t>(pix.n) * 3 + c) * oh + (2 * pix.y + py)) * ow + 2 * pix.x;
             *reinterpret_cast<float2*>(dst) = o;
           }
         }
       }
     } else {
       constexpr int kPieces = BN / 32;             // 32-column pieces of the tile; this warp takes grp, grp+kGroups, ...
-      if (split_mode && CSP) {
-        // ---- cluster split-K: this thread's fp32 accumulator row goes to the CTA that owns the row (distributed shared
-        // memory), into the slot of this CTA's rank; cluster_split_finish() sums the slots after the cluster barrier.
-        const int rpo = kTileM / p.n_split;                      // rows per owner
-        const uint32_t owner = static_cast<uint32_t>(row / rpo);
-        const int lr = row - static_cast<int>(owner) * rpo;
-        const uint32_t my_rank = ptx::cluster_ctarank();
-        const uint32_t dst = ptx::mapa_u32(ptx::smem_u32(stg_base) + ((my_rank * rpo + lr) * BN) * 4u, owner);
-#pragma unroll 1
-        for (int c32 = grp; c32 < kPieces; c32 += kGroups) {
-          uint32_t v[32];
-          ptx::tmem_ld_32x32(t_acc + c32 * 32, v);
-          if constexpr (STACK) {
-            uint32_t v2[32];
-            ptx::tmem_ld_32x32(t_acc + BN + c32 * 32, v2);
-            ptx::tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(__uint_as_float(v[i]) + __uint_as_float(v2[i]));
-          }
-          ptx::tmem_ld_wait();
-          if (c32 + kGroups >= kPieces) release_tmem();
-#pragma unroll
-          for (int e = 0; e < 8; ++e)
-            ptx::st_cluster_v4(dst + (c32 * 32 + e * 4) * 4u, v[4 * e], v[4 * e + 1], v[4 * e + 2], v[4 * e + 3]);
-        }
-      } else if (split_mode) {
-        // ---- split-K partial: raw fp32 accumulator rows -> partial[t][row][BN]
+      if (split_mode) {
+        // ---- split-K: this thread's raw fp32 accumulator row.  CSP: into the slot of this CTA's rank in the staging buffer
+        // of the CTA that owns the row (distributed shared memory); cluster_split_finish() sums the slots after the cluster
+        // barrier.  Otherwise: to partial[t][row][BN] in global memory, summed by splitk_reduce_kernel.
+        uint32_t dst_cl = 0;
         float* dst = p.partial + (static_cast<size_t>(t) * kTileM + row) * BN;
+        if constexpr (CSP) {
+          const int rpo = kTileM / p.n_split;                      // rows per owner
+          const uint32_t owner = static_cast<uint32_t>(row / rpo);
+          const int lr = row - static_cast<int>(owner) * rpo;
+          const uint32_t my_rank = ptx::cluster_ctarank();
+          dst_cl = ptx::mapa_u32(ptx::smem_u32(stg_base) + ((my_rank * rpo + lr) * BN) * 4u, owner);
+        }
 #pragma unroll 1
         for (int c32 = grp; c32 < kPieces; c32 += kGroups) {
           uint32_t v[32];
@@ -426,37 +469,39 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
           ptx::tmem_ld_wait();
           if (c32 + kGroups >= kPieces) release_tmem();
 #pragma unroll
-          for (int e = 0; e < 8; ++e)
-            *reinterpret_cast<uint4*>(dst + c32 * 32 + e * 4) = make_uint4(v[4 * e], v[4 * e + 1], v[4 * e + 2], v[4 * e + 3]);
+          for (int e = 0; e < 8; ++e) {
+            if constexpr (CSP)
+              ptx::st_cluster_v4(dst_cl + (c32 * 32 + e * 4) * 4u, v[4 * e], v[4 * e + 1], v[4 * e + 2], v[4 * e + 3]);
+            else
+              *reinterpret_cast<uint4*>(dst + c32 * 32 + e * 4) = make_uint4(v[4 * e], v[4 * e + 1], v[4 * e + 2], v[4 * e + 3]);
+          }
         }
       } else {
-        // ---- regular: scale/shift (+ residual) + ReLU, bf16 (hi, lo), written straight to the NHWC output.
+        // ---- regular: scale/shift (+ residual) + ReLU, 16-bit (hi, lo), written straight to the NHWC output.
         // Each thread owns one pixel row; per 32-column piece it reads its residual (64 B per limb) and writes its output
         // with 256-bit (one 32-byte sector) global accesses.  No smem staging and no TMA store: a TMA store queues behind
         // the producer's outstanding TMA loads in the SM's TMA pipe (measured ~3 us per chunk), and global stores are
         // fire-and-forget.
-        const int oh = p.out_up ? 2 * p.hs : p.hs, ow = p.out_up ? 2 * p.ws : p.ws;
-        const int oy = p.out_up ? 2 * py_ + (tc.z >> 1) : py_, ox = p.out_up ? 2 * px_ + (tc.z & 1) : px_;
-        __nv_bfloat16* out_row = p.out_ptr + ((static_cast<size_t>(pn) * oh + oy) * ow + ox) * p.out_channels + tc.nt * BN;
+        const OutPixel pix = out_pixel(p, tc, row);
+        __nv_bfloat16* out_row = p.out_ptr + pix.out + tc.nt * BN;
 #pragma unroll 1
         for (int c32 = grp; c32 < kPieces; c32 += kGroups) {
           uint32_t vv[32];
-          {
-            ptx::tmem_ld_32x32(t_acc + c32 * 32, vv);
-            if constexpr (STACK) {
-              // second half of the stacked accumulator, 16 columns at a time (register pressure: 168 per thread at 10 warps)
+          ptx::tmem_ld_32x32(t_acc + c32 * 32, vv);
+          if constexpr (STACK) {
+            // second half of the stacked accumulator 16 columns at a time (register pressure: 168 per thread at 10 warps;
+            // even a force-inlined helper shared with the split-K branch above costs patch<128, NL=2> 20 more spill bytes)
 #pragma unroll
-              for (int hh = 0; hh < 2; ++hh) {
-                uint32_t v2[16];
-                ptx::tmem_ld_32x16(t_acc + BN + c32 * 32 + hh * 16, v2);
-                ptx::tmem_ld_wait();
+            for (int hh = 0; hh < 2; ++hh) {
+              uint32_t v2[16];
+              ptx::tmem_ld_32x16(t_acc + BN + c32 * 32 + hh * 16, v2);
+              ptx::tmem_ld_wait();
 #pragma unroll
-                for (int i = 0; i < 16; ++i) vv[hh * 16 + i] = __float_as_uint(__uint_as_float(vv[hh * 16 + i]) + __uint_as_float(v2[i]));
-              }
+              for (int i = 0; i < 16; ++i) vv[hh * 16 + i] = __float_as_uint(__uint_as_float(vv[hh * 16 + i]) + __uint_as_float(v2[i]));
             }
-            ptx::tmem_ld_wait();
-            if (c32 + kGroups >= kPieces) release_tmem();   // this warp's share of the accumulator is in registers
           }
+          ptx::tmem_ld_wait();
+          if (c32 + kGroups >= kPieces) release_tmem();   // this warp's share of the accumulator is in registers
           // this piece's residual was requested one piece ahead.  A warp with several pieces per tile keeps two register
           // sets (the next request is issued before the math); with one piece per tile the next request - the next TILE's
           // residual, a whole tile period ahead of its use - is issued after the math into the same registers.
@@ -481,37 +526,16 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
               const int ch = c32 * 32 + piece * 8 + e;
               y[e] = fmaf(__uint_as_float(vv[piece * 8 + e]), s_scale[ch], s_shift[ch]);
             }
-            if (p.has_res) {
+            uint32_t r[NL][4], hi[4], lo[4];
 #pragma unroll
-              for (int l = 0; l < NL; ++l) {
-                const uint32_t rr[4] = {rc[l][piece].x, rc[l][piece].y, rc[l][piece].z, rc[l][piece].w};
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  y[2 * e] += unpack_lo<NL == 2>(rr[e]);
-                  y[2 * e + 1] += unpack_hi<NL == 2>(rr[e]);
-                }
-              }
+            for (int l = 0; l < NL; ++l) {
+              r[l][0] = rc[l][piece].x; r[l][1] = rc[l][piece].y; r[l][2] = rc[l][piece].z; r[l][3] = rc[l][piece].w;
             }
-            if (p.relu) {
-#pragma unroll
-              for (int e = 0; e < 8; ++e) y[e] = fmaxf(y[e], 0.0f);
-            }
-            uint4 o;
-            o.x = pack2<NL == 2>(y[0], y[1]);
-            o.y = pack2<NL == 2>(y[2], y[3]);
-            o.z = pack2<NL == 2>(y[4], y[5]);
-            o.w = pack2<NL == 2>(y[6], y[7]);
-            uint4 ol = make_uint4(0u, 0u, 0u, 0u);
-            if (NL == 2) {
-              const uint32_t oo[4] = {o.x, o.y, o.z, o.w};
-              uint32_t lo[4];
-#pragma unroll
-              for (int e = 0; e < 4; ++e)
-                lo[e] = pack2<true>(y[2 * e] - unpack_lo<true>(oo[e]), y[2 * e + 1] - unpack_hi<true>(oo[e]));
-              ol = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-            }
+            finish_channels<NL, 8>(y, r, p.has_res, p.relu, hi, lo);
+            const uint4 o = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+            const uint4 ol = NL == 2 ? make_uint4(lo[0], lo[1], lo[2], lo[3]) : make_uint4(0u, 0u, 0u, 0u);
             if (piece & 1) {               // two 16-byte pieces = one 32-byte sector per store
-              if (pix_ok) {
+              if (pix.ok) {
                 ptx::stg256(out_row + c32 * 32 + (piece - 1) * 8, o_prev, o);
                 if (NL == 2) ptx::stg256(out_row + p.out_limb_stride + c32 * 32 + (piece - 1) * 8, ol_prev, ol);
               }
@@ -532,8 +556,8 @@ __device__ __forceinline__ void epilogue_warps(const ConvParams& p, uint8_t* stg
 }
 
 // Cluster split-K, second half (after the cluster barrier): the epilogue warps of every CTA sum the n_split partial slots of
-// the 128 / n_split tile rows this CTA owns (in split order: deterministic) and apply the layer's epilogue - folded BatchNorm,
-// residual, ReLU, 16-bit hi/lo split - writing the NHWC output directly.  One thread = one pixel x 4 channels per trip.
+// the 128 / n_split tile rows this CTA owns (in split order: deterministic) and finish them (finish4), writing the NHWC output
+// directly.  One thread = one pixel x 4 channels per trip.
 template <int BN, int NL, int EW>
 __device__ __forceinline__ void cluster_split_finish(const ConvParams& p, const uint8_t* stg_base, int t) {
   constexpr int kEpi = EW * 32;
@@ -545,45 +569,14 @@ __device__ __forceinline__ void cluster_split_finish(const ConvParams& p, const 
   constexpr int kGroups4 = BN / 4;
   for (int e = etid; e < rpo * kGroups4; e += kEpi) {
     const int g = e % kGroups4, lr = e / kGroups4;
-    const int row = rank * rpo + lr;
-    const int tw_ = row & ((1 << p.tw_log2) - 1);
-    const int th_ = (row >> p.tw_log2) & ((1 << p.th_log2) - 1);
-    const int nb_ = row >> (p.tw_log2 + p.th_log2);
-    const int n = tc.n0 + nb_, y = tc.y0 + th_, x = tc.x0 + tw_;
-    if (n >= p.batch || y >= p.hs || x >= p.ws) continue;
+    const OutPixel pix = out_pixel(p, tc, rank * rpo + lr);
+    if (!pix.ok) continue;
     float4 acc = *reinterpret_cast<const float4*>(stg + (static_cast<size_t>(lr) * BN + g * 4));
     for (int sp = 1; sp < cs; ++sp) {
       const float4 a = *reinterpret_cast<const float4*>(stg + (static_cast<size_t>(sp * rpo + lr) * BN + g * 4));
       acc.x += a.x; acc.y += a.y; acc.z += a.z; acc.w += a.w;
     }
-    const int ch = tc.nt * BN + g * 4;
-    const float4 sc = *reinterpret_cast<const float4*>(p.scale + ch), sh = *reinterpret_cast<const float4*>(p.shift + ch);
-    float yv[4] = {fmaf(acc.x, sc.x, sh.x), fmaf(acc.y, sc.y, sh.y), fmaf(acc.z, sc.z, sh.z), fmaf(acc.w, sc.w, sh.w)};
-    if (p.has_res) {
-      const __nv_bfloat16* rr = p.res_ptr + ((static_cast<size_t>(n) * p.hs + y) * p.ws + x) * p.res_channels + ch;
-#pragma unroll
-      for (int l = 0; l < NL; ++l) {
-        const uint2 r = *reinterpret_cast<const uint2*>(rr + l * p.res_limb_stride);
-        yv[0] += unpack_lo<NL == 2>(r.x); yv[1] += unpack_hi<NL == 2>(r.x);
-        yv[2] += unpack_lo<NL == 2>(r.y); yv[3] += unpack_hi<NL == 2>(r.y);
-      }
-    }
-    if (p.relu) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) yv[i] = fmaxf(yv[i], 0.f);
-    }
-    const int oh = p.out_up ? 2 * p.hs : p.hs, ow = p.out_up ? 2 * p.ws : p.ws;
-    const int oy = p.out_up ? 2 * y + (tc.z >> 1) : y, ox = p.out_up ? 2 * x + (tc.z & 1) : x;
-    __nv_bfloat16* out = p.out_ptr + ((static_cast<size_t>(n) * oh + oy) * ow + ox) * p.out_channels + ch;
-    uint2 o;
-    o.x = pack2<NL == 2>(yv[0], yv[1]); o.y = pack2<NL == 2>(yv[2], yv[3]);
-    *reinterpret_cast<uint2*>(out) = o;
-    if (NL == 2) {
-      uint2 lo;
-      lo.x = pack2<true>(yv[0] - unpack_lo<true>(o.x), yv[1] - unpack_hi<true>(o.x));
-      lo.y = pack2<true>(yv[2] - unpack_lo<true>(o.y), yv[3] - unpack_hi<true>(o.y));
-      *reinterpret_cast<uint2*>(out + p.out_limb_stride) = lo;
-    }
+    finish4<NL>(p, pix, tc.nt * BN + g * 4, acc);
   }
 }
 
@@ -613,14 +606,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
   uint8_t* stg_base = smem + Cfg::kStages * Cfg::kStage;
   uint8_t* aux = stg_base + Cfg::kStgBytes;
   float* s_scale = reinterpret_cast<float*>(aux);
-  float* s_shift = s_scale + BN;
   uint64_t* bars = reinterpret_cast<uint64_t*>(aux + 4 * BN * 4);
   uint64_t* full_bar = bars;                       // [kStages]
   uint64_t* empty_bar = bars + Cfg::kStages;       // [kStages]
   uint64_t* tfull_bar = bars + 2 * Cfg::kStages;   // [2]
   uint64_t* tempty_bar = tfull_bar + 2;            // [2]
-  uint64_t* stg_bar = tempty_bar + 2;              // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(stg_bar + 2);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
 
   const int warp = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);   // provably warp-uniform
   const int lane = threadIdx.x & 31;
@@ -628,9 +619,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < 4; ++i) ptx::prefetch_tmap(&p.a[i]);
     ptx::prefetch_tmap(&p.w);
-    if (!TAIL) {
-      for (int i = 0; i < 4; ++i) ptx::prefetch_tmap(&p.out[i]);
-    }
     for (int i = 0; i < Cfg::kStages; ++i) {
       ptx::mbar_init(&full_bar[i], 1);
       ptx::mbar_init(&empty_bar[i], 1);
@@ -638,7 +626,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
     for (int i = 0; i < 2; ++i) {
       ptx::mbar_init(&tfull_bar[i], 1);
       ptx::mbar_init(&tempty_bar[i], 4);   // one arrive per epilogue warp
-      ptx::mbar_init(&stg_bar[i], 1);
     }
     ptx::fence_mbar_init();
   }
@@ -755,8 +742,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
   } else {
-    epilogue_warps<BN, NL, TAIL, Cfg::kNumStg, false, false, 4, 2, CSP>(p, stg_base, s_scale, s_shift, tfull_bar, tempty_bar, stg_bar,
-                                                                         tmem_base, warp, lane, t0, tstep);
+    epilogue_warps<BN, NL, TAIL, false, false, 4, 2, CSP>(p, stg_base, s_scale, tfull_bar, tempty_bar, tmem_base, warp, lane,
+                                                           t0, tstep);
   }
   if constexpr (CSP) {
     // every CTA of the cluster has written its partial rows into the owners' staging buffers
@@ -781,18 +768,24 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
 // one image row of the patch, so the shifted A tile of tap (dx,dy) is the same swizzled buffer described by
 //   start = patch + ((dy-dy0)*PW + (dx-dx0)) * 128 B,   stride between 8-row groups (SBO) = PW * 128 B.
 // The swizzle phase of a row is a function of its absolute smem address for both TMA and UMMA, so rows that
-// TMA wrote are read back consistently at any 128-byte-aligned start (descriptor base offset = (start>>7)&7).
+// TMA wrote are read back consistently at any 128-byte-aligned start with a descriptor base offset of 0 (measured on
+// B200: setting it to (start>>7)&7 corrupts the result).
 // A and B move through separate mbarrier rings: an A patch is consumed by n_taps B tiles.
 // ====================================================================================================
 constexpr int kPatchSlot = 23 * 1024;           // >= 10*18*128 = 23040 bytes
 constexpr int kPatchStride = 23 * 1024;         // distance between patch buffers (1024-byte aligned)
 
+// Taps per B stage of conv_patch_kernel (build_plan encodes the FAST single-CTA weight view with boxes of this many taps):
+// one mbarrier round trip per stage costs the MMA-issuing thread a few hundred cycles, so a stage must carry enough tensor
+// work (>= ~500 cycles): 2 taps for N=128 bf16, 2-3 for N=64, all 9 for the tail.
+constexpr int patch_taps_per_stage(int bn, int nl, bool tail) {
+  return tail ? 9 : (bn >= 128 ? (nl == 1 ? 2 : 1) : (nl == 1 ? 3 : 2));
+}
+
 template <int BN, int NL, bool TAIL, bool CSP = false>
 struct PatchCfg {
   static constexpr int kBTile = BN * 128;
-  // taps per B stage: one mbarrier round trip per stage costs the MMA-issuing thread a few hundred cycles, so a
-  // stage must carry enough tensor work (>= ~500 cycles): 2 taps for N=128 bf16, 2-3 for N=64, all 9 for the tail.
-  static constexpr int kTPS = TAIL ? 9 : (BN >= 128 ? (NL == 1 ? 2 : 1) : (NL == 1 ? 3 : 2));
+  static constexpr int kTPS = patch_taps_per_stage(BN, NL, TAIL);
   static constexpr int kAStage = NL * kPatchStride;
   static constexpr int kBStage = NL * kTPS * kBTile;
   // In-kernel clock64 traces (tests/gpu_trace.py) showed the MMA warp stalling ~350 cycles per B stage: a stage is
@@ -800,7 +793,6 @@ struct PatchCfg {
   // ~2.3-2.7k cycles, so the B ring must hold more than that much tensor work.  Two A patches are enough (the next
   // one is requested a full chunk ahead); everything else goes to B stages.
   static constexpr int kAStages = 2;
-  static constexpr int kNumStg = 0;
   static constexpr int kStgBytes = CSP ? kTileM * BN * 4 : 0;        // cluster split-K staging (see ConvCfg)
   static constexpr int kAux = 3072;
   static constexpr int kAvail = kSmemBudget - 1024 - kStgBytes - kAux - kAStages * kAStage;
@@ -811,16 +803,15 @@ struct PatchCfg {
   static constexpr int kTmemCols = (2 * kAccCols < 32) ? 32 : 2 * kAccCols;
   static_assert(kTmemCols <= 512, "TMEM has 512 columns");
   static_assert(kBStages >= 2, "B ring needs at least two stages");
-  static_assert(4 * BN * 4 + (2 * 12 + 2 * 2 + 8) * 8 <= kAux, "aux region too small");
+  static_assert(4 * BN * 4 + (2 * kBStages + 2 * kAStages + 2 * 2 + 1) * 8 <= kAux, "aux region too small");
 };
 
-__device__ __forceinline__ uint64_t umma_desc_sw128_strided(uint32_t smem_addr, uint32_t sbo_bytes, bool base_off) {
+__device__ __forceinline__ uint64_t umma_desc_sw128_strided(uint32_t smem_addr, uint32_t sbo_bytes) {
   uint64_t d = 0;
   d |= static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4);
   d |= static_cast<uint64_t>(1) << 16;
   d |= static_cast<uint64_t>(sbo_bytes >> 4) << 32;
   d |= static_cast<uint64_t>(1) << 46;
-  if (base_off) d |= static_cast<uint64_t>((smem_addr >> 7) & 7u) << 49;
   d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
@@ -843,7 +834,6 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
   uint8_t* stg_base = b_ring + Cfg::kBStages * Cfg::kBStage;
   uint8_t* aux = stg_base + Cfg::kStgBytes;
   float* s_scale = reinterpret_cast<float*>(aux);
-  float* s_shift = s_scale + BN;
   uint64_t* bars = reinterpret_cast<uint64_t*>(aux + 4 * BN * 4);
   uint64_t* afull_bar = bars;                               // [kAStages]
   uint64_t* aempty_bar = afull_bar + Cfg::kAStages;         // [kAStages]
@@ -851,8 +841,7 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
   uint64_t* bempty_bar = bfull_bar + Cfg::kBStages;         // [kBStages]
   uint64_t* tfull_bar = bempty_bar + Cfg::kBStages;         // [2]
   uint64_t* tempty_bar = tfull_bar + 2;                     // [2]
-  uint64_t* stg_bar = tempty_bar + 2;                       // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(stg_bar + 2);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
 
   const int warp = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);   // provably warp-uniform
   const int lane = threadIdx.x & 31;
@@ -861,15 +850,11 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < 4; ++i) ptx::prefetch_tmap(&p.a[i]);
     ptx::prefetch_tmap(&p.w);
-    if (!TAIL) {
-      for (int i = 0; i < 4; ++i) ptx::prefetch_tmap(&p.out[i]);
-    }
     for (int i = 0; i < Cfg::kAStages; ++i) { ptx::mbar_init(&afull_bar[i], 1); ptx::mbar_init(&aempty_bar[i], 1); }
     for (int i = 0; i < Cfg::kBStages; ++i) { ptx::mbar_init(&bfull_bar[i], 1); ptx::mbar_init(&bempty_bar[i], CL); }
     for (int i = 0; i < 2; ++i) {
       ptx::mbar_init(&tfull_bar[i], 1);
       ptx::mbar_init(&tempty_bar[i], EW);   // one arrive per epilogue warp
-      ptx::mbar_init(&stg_bar[i], 1);
     }
     ptx::fence_mbar_init();
   }
@@ -971,7 +956,6 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
     int acc = 0;
     uint32_t acc_phase = 0;
     const uint32_t sbo = static_cast<uint32_t>(p.patch_w) * 128u;
-    const bool boff = p.desc_base_offset != 0;
     const int n_groups = (p.n_taps + Cfg::kTPS - 1) / Cfg::kTPS;
     bool b_ready = false;
     int lt = 0;
@@ -998,7 +982,7 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
             for (int tap = tap0; tap < tap1; ++tap) {
               const uint32_t a_hi_addr = a0 + static_cast<uint32_t>(p.tap_row[tc.z][tap]) * 128u;
               const uint32_t b_hi_addr = b0 + static_cast<uint32_t>(tap - tap0) * (NL * Cfg::kBTile);
-              const uint64_t a_hi = umma_desc_sw128_strided(a_hi_addr, sbo, boff);
+              const uint64_t a_hi = umma_desc_sw128_strided(a_hi_addr, sbo);
               const uint64_t b_hi = ptx::umma_desc_sw128(b_hi_addr);
 #pragma unroll
               for (int k = 0; k < kChunk / 16; ++k) {
@@ -1007,7 +991,7 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
                   ptx::umma_f16(d_tmem, a_hi + 2 * k, b_hi + 2 * k, p.idesc, accum);
                 } else {
                   // [hi*hi | hi*lo] in one N=2*BN MMA (B_lo is stored right behind B_hi), then lo*hi into the first half
-                  const uint64_t a_lo = umma_desc_sw128_strided(a_hi_addr + kPatchStride, sbo, boff);
+                  const uint64_t a_lo = umma_desc_sw128_strided(a_hi_addr + kPatchStride, sbo);
                   ptx::umma_f16(d_tmem, a_hi + 2 * k, b_hi + 2 * k, p.idesc2, accum);
                   ptx::umma_f16(d_tmem, a_lo + 2 * k, b_hi + 2 * k, p.idesc, 1u);
                 }
@@ -1030,8 +1014,8 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
   } else {
-    epilogue_warps<BN, NL, TAIL, Cfg::kNumStg, (NL == 2), false, EW, 2, CSP>(p, stg_base, s_scale, s_shift, tfull_bar, tempty_bar, stg_bar,
-                                                                              tmem_base, warp, lane, t0, tstep);
+    epilogue_warps<BN, NL, TAIL, (NL == 2), false, EW, 2, CSP>(p, stg_base, s_scale, tfull_bar, tempty_bar, tmem_base, warp, lane,
+                                                                t0, tstep);
   }
   if constexpr (CSP) {
     ptx::cluster_sync();                 // every CTA's partial rows are in their owners' staging buffers
@@ -1061,18 +1045,29 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_patch_kernel(const __gri
 // stacked [B_hi; B_lo] operand of one N = 128 MMA: A_hi*B_hi | A_hi*B_lo) and Y = rows [32r, 32r+32) of B_hi (the pair's
 // Y tiles form B_hi for the N = 64 MMA A_lo*B_hi).  Two MMAs instead of three per K step and 11 KB instead of 15 KB of
 // operand reads per SM: the N = 64 layers are bound by shared-memory bandwidth (A is re-read for every 64 columns).
-template <int BN, int NL, bool STK = false>
+constexpr bool pair_stacked(int bn, int nl) { return bn == 64 && nl == 2; }
+
+// Shared memory of the pair kernel: two A patches, the aux region and a B ring of one tap per stage (this CTA's half of the
+// B tile of every limb; three halves when stacked) that takes the rest, at most 16 stages.  build_plan keeps a layer's
+// weights resident when all of its weight tiles fit that ring.
+constexpr int kPairAStages = 2;
+constexpr int kPairAux = 5120;
+constexpr int pair_b_stage_bytes(int bn, int nl) { return (pair_stacked(bn, nl) ? 3 : nl) * (bn / 2) * 128; }
+constexpr int pair_b_stages(int bn, int nl) {
+  const int n = (kSmemBudget - 1024 - kPairAux - kPairAStages * nl * kPatchStride) / pair_b_stage_bytes(bn, nl);
+  return n > 16 ? 16 : n;
+}
+
+template <int BN, int NL, bool STK>
 struct PairCfg {
-  static_assert(!STK || (NL == 2 && BN == 64), "stacked operands: parity mode, N tile 64");
+  static_assert(STK == pair_stacked(BN, NL), "stacked operands exactly in parity mode with N tile 64");
   static constexpr int kBHalf = (BN / 2) * 128;                   // bytes of this CTA's half of one B tile
   static constexpr int kAStage = NL * kPatchStride;
-  static constexpr int kBStage = STK ? 3 * kBHalf : NL * kBHalf;  // one tap per stage
+  static constexpr int kBStage = pair_b_stage_bytes(BN, NL);
   static constexpr int kAccCols = STK ? 2 * BN : BN;
-  static constexpr int kAStages = 2;
-  static constexpr int kAux = 5120;
-  static constexpr int kAvail = kSmemBudget - 1024 - kAux - kAStages * kAStage;
-  static constexpr int kBStagesRaw = kAvail / kBStage;
-  static constexpr int kBStages = kBStagesRaw > 16 ? 16 : kBStagesRaw;
+  static constexpr int kAStages = kPairAStages;
+  static constexpr int kAux = kPairAux;
+  static constexpr int kBStages = pair_b_stages(BN, NL);
   static constexpr int kSmemBytes = 1024 + kAStages * kAStage + kBStages * kBStage + kAux;
   // TMEM accumulator ring: as many buffers as the 512 columns hold (4 for N tiles up to 128 columns wide, 2 for 256).
   // With two buffers the MMA warp idled ~15 % of a 64-channel tile waiting for the epilogue to hand one back (clock64
@@ -1082,10 +1077,10 @@ struct PairCfg {
   static_assert(BN == 64 || BN == 128 || BN == 256, "pair kernel: N tile 64, 128 or 256");
   static_assert(kTmemCols <= 512, "TMEM has 512 columns");
   static_assert(kBStages >= 3, "B ring too shallow");
-  static_assert(4 * BN * 4 + (2 * 16 + 3 * 4 + 8) * 8 <= kAux, "aux region too small");
+  static_assert(4 * BN * 4 + (2 * kBStages + 2 * kAStages + 2 * kAccBufs + 1) * 8 <= kAux, "aux region too small");
 };
 
-template <int BN, int NL, int EW, bool STK = false>
+template <int BN, int NL, int EW, bool STK>
 __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid_constant__ ConvParams p) {
   using Cfg = PairCfg<BN, NL, STK>;
   extern __shared__ uint8_t smem_raw[];
@@ -1094,7 +1089,6 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid
   uint8_t* b_ring = a_ring + Cfg::kAStages * Cfg::kAStage;
   uint8_t* aux = b_ring + Cfg::kBStages * Cfg::kBStage;
   float* s_scale = reinterpret_cast<float*>(aux);
-  float* s_shift = s_scale + BN;
   uint64_t* bars = reinterpret_cast<uint64_t*>(aux + 4 * BN * 4);
   uint64_t* afull_bar = bars;                               // [kAStages]  (used in the leader)
   uint64_t* aempty_bar = afull_bar + Cfg::kAStages;         // [kAStages]
@@ -1103,8 +1097,7 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid
   constexpr int NACC = Cfg::kAccBufs;
   uint64_t* tfull_bar = bempty_bar + Cfg::kBStages;         // [NACC]
   uint64_t* tempty_bar = tfull_bar + NACC;                  // [NACC]     (used in the leader: 2*EW arrivals)
-  uint64_t* stg_bar = tempty_bar + NACC;                    // [2] unused (layout shared with the other kernels)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(stg_bar + 2);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + NACC);
 
   const int warp = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
@@ -1121,7 +1114,6 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid
       ptx::mbar_init(&tfull_bar[i], 1);
       ptx::mbar_init(&tempty_bar[i], 2 * EW);  // the epilogue warps of both CTAs of the pair
     }
-    for (int i = 0; i < 2; ++i) ptx::mbar_init(&stg_bar[i], 1);
     ptx::fence_mbar_init();
   }
   if (warp == 1) {
@@ -1268,20 +1260,20 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid
             if (ptx::elect_one()) {
               const uint32_t b0 = ptx::smem_u32(b_ring + (resident ? ci * p.n_taps + tap : ib) * Cfg::kBStage);
               const uint32_t a_hi_addr = a0 + static_cast<uint32_t>(p.tap_row[z][tap]) * 128u;
-              const uint64_t a_hi = umma_desc_sw128_strided(a_hi_addr, sbo, false);
+              const uint64_t a_hi = umma_desc_sw128_strided(a_hi_addr, sbo);
               const uint64_t b_hi = ptx::umma_desc_sw128(b0);
 #pragma unroll
               for (int k = 0; k < kChunk / 16; ++k) {
                 const uint32_t accum = (ci > 0 || tap > 0 || k > 0) ? 1u : 0u;
                 if constexpr (STK) {
-                  const uint64_t a_lo = umma_desc_sw128_strided(a_hi_addr + kPatchStride, sbo, false);
+                  const uint64_t a_lo = umma_desc_sw128_strided(a_hi_addr + kPatchStride, sbo);
                   const uint64_t b_y = ptx::umma_desc_sw128(b0 + 2 * Cfg::kBHalf);
                   ptx::umma_f16_pair(d_tmem, a_hi + 2 * k, b_hi + 2 * k, p.idesc2, accum);   // N = 2*BN: A_hi*[B_hi | B_lo]
                   ptx::umma_f16_pair(d_tmem, a_lo + 2 * k, b_y + 2 * k, p.idesc, 1u);        // N = BN:   A_lo*B_hi
                 } else {
                 ptx::umma_f16_pair(d_tmem, a_hi + 2 * k, b_hi + 2 * k, p.idesc, accum);
                 if (NL == 2) {
-                  const uint64_t a_lo = umma_desc_sw128_strided(a_hi_addr + kPatchStride, sbo, false);
+                  const uint64_t a_lo = umma_desc_sw128_strided(a_hi_addr + kPatchStride, sbo);
                   const uint64_t b_lo = ptx::umma_desc_sw128(b0 + Cfg::kBHalf);
                   ptx::umma_f16_pair(d_tmem, a_hi + 2 * k, b_lo + 2 * k, p.idesc, 1u);
                   ptx::umma_f16_pair(d_tmem, a_lo + 2 * k, b_hi + 2 * k, p.idesc, 1u);
@@ -1307,8 +1299,8 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid
       }
     }
   } else {
-    epilogue_warps<BN, NL, false, 0, STK, true, EW, NACC>(p, aux, s_scale, s_shift, tfull_bar, tempty_bar, stg_bar, tmem_base, warp, lane,
-                                                          static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x));
+    epilogue_warps<BN, NL, false, STK, true, EW, NACC>(p, nullptr, s_scale, tfull_bar, tempty_bar, tmem_base, warp, lane,
+                                                       static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x));
   }
 
   ptx::tc_fence_before();
@@ -1322,29 +1314,18 @@ __global__ void __launch_bounds__(64 + EW * 32, 1) conv_pair_kernel(const __grid
 }
 
 // ====================================================================================================
-// Split-K finisher: out = epilogue( sum_s partial[s] ).
+// Split-K finisher: out = epilogue( sum_s partial[s] ), for the layer's ConvParams and N tile `bn`.
 // Memory-bound and tiny (the layers that use split-K have at most a few hundred output pixels per image).
 // ====================================================================================================
-struct ReduceParams {
-  const float* partial;
-  const float* scale;
-  const float* shift;
-  const __nv_bfloat16* res;
-  long long res_limb_stride;      // elements
-  __nv_bfloat16* out;
-  long long out_limb_stride;
-  int32_t n_split, tiles_per_split, m_tiles, n_tiles, n_phases;
-  int32_t tiles_x, tiles_y, tw_log2, th_log2, bn;
-  int32_t batch, hs, ws, up, channels, relu, has_res, nl;
-};
-
-// One thread = one pixel x 4 channels.  The layers that use split-K are latency bound (a few hundred output pixels, 8-36
-// splits): what matters is how many dependent trips to L2 the sum takes, so up to 16 splits are in flight per trip
-// (round 1 summed 4 per trip over 8-channel groups: 6 dependent trips for 18 splits, as long as the conv itself at batch 1).
-__global__ void __launch_bounds__(128) splitk_reduce_kernel(const ReduceParams p) {
+// One thread = one pixel x 4 channels of a split-0 tile t (0 <= t < tiles_per_split).  The layers that use split-K are
+// latency bound (a few hundred output pixels, 8-36 splits): what matters is how many dependent trips to L2 the sum takes, so
+// up to 16 splits are in flight per trip (round 1 summed 4 per trip over 8-channel groups: 6 dependent trips for 18 splits,
+// as long as the conv itself at batch 1).
+template <int NL>
+__global__ void __launch_bounds__(128) splitk_reduce_kernel(const __grid_constant__ ConvParams p, int bn) {
   ptx::pdl_wait();
   ptx::pdl_launch_dependents();
-  const int groups = p.bn >> 2;
+  const int groups = bn >> 2;
   const long long total = static_cast<long long>(p.tiles_per_split) * kTileM * groups;
   for (long long e = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; e < total;
        e += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -1352,23 +1333,12 @@ __global__ void __launch_bounds__(128) splitk_reduce_kernel(const ReduceParams p
     const long long r0 = e / groups;
     const int row = static_cast<int>(r0 % kTileM);
     const int tile = static_cast<int>(r0 / kTileM);
-    const int mt = tile % p.m_tiles;
-    const int r1 = tile / p.m_tiles;
-    const int nt = r1 % p.n_tiles;
-    const int z = r1 / p.n_tiles;
-    const int tx = mt % p.tiles_x;
-    const int r2 = mt / p.tiles_x;
-    const int ty = r2 % p.tiles_y;
-    const int tn = r2 / p.tiles_y;
-    const int tw = row & ((1 << p.tw_log2) - 1);
-    const int th = (row >> p.tw_log2) & ((1 << p.th_log2) - 1);
-    const int nb = row >> (p.tw_log2 + p.th_log2);
-    const int n = (tn << (7 - p.tw_log2 - p.th_log2)) + nb;
-    const int y = (ty << p.th_log2) + th, x = (tx << p.tw_log2) + tw;
-    if (n >= p.batch || y >= p.hs || x >= p.ws) continue;
-    float acc[4] = {0.f, 0.f, 0.f, 0.f};
-    const size_t split_stride = static_cast<size_t>(p.tiles_per_split) * kTileM * p.bn;      // floats between splits
-    const float* src0 = p.partial + (static_cast<size_t>(tile) * kTileM + row) * p.bn + g * 4;
+    const TileCoord tc = decode_tile(p, tile);
+    const OutPixel pix = out_pixel(p, tc, row);
+    if (!pix.ok) continue;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    const size_t split_stride = static_cast<size_t>(p.tiles_per_split) * kTileM * bn;      // floats between splits
+    const float* src0 = p.partial + (static_cast<size_t>(tile) * kTileM + row) * bn + g * 4;
     int s = 0;
     for (; s + 16 <= p.n_split; s += 16) {     // sixteen independent 16-byte loads in flight
       float4 v[16];
@@ -1376,7 +1346,7 @@ __global__ void __launch_bounds__(128) splitk_reduce_kernel(const ReduceParams p
       for (int u = 0; u < 16; ++u) v[u] = *reinterpret_cast<const float4*>(src0 + (s + u) * split_stride);
 #pragma unroll
       for (int u = 0; u < 16; ++u) {           // summation order stays s = 0, 1, 2, ... (deterministic)
-        acc[0] += v[u].x; acc[1] += v[u].y; acc[2] += v[u].z; acc[3] += v[u].w;
+        acc.x += v[u].x; acc.y += v[u].y; acc.z += v[u].z; acc.w += v[u].w;
       }
     }
     for (; s + 4 <= p.n_split; s += 4) {
@@ -1384,44 +1354,13 @@ __global__ void __launch_bounds__(128) splitk_reduce_kernel(const ReduceParams p
 #pragma unroll
       for (int u = 0; u < 4; ++u) v[u] = *reinterpret_cast<const float4*>(src0 + (s + u) * split_stride);
 #pragma unroll
-      for (int u = 0; u < 4; ++u) { acc[0] += v[u].x; acc[1] += v[u].y; acc[2] += v[u].z; acc[3] += v[u].w; }
+      for (int u = 0; u < 4; ++u) { acc.x += v[u].x; acc.y += v[u].y; acc.z += v[u].z; acc.w += v[u].w; }
     }
     for (; s < p.n_split; ++s) {
       const float4 a = *reinterpret_cast<const float4*>(src0 + s * split_stride);
-      acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
+      acc.x += a.x; acc.y += a.y; acc.z += a.z; acc.w += a.w;
     }
-    const int ch = nt * p.bn + g * 4;
-    const int oh = p.up ? 2 * p.hs : p.hs, ow = p.up ? 2 * p.ws : p.ws;
-    const int oy = p.up ? 2 * y + (z >> 1) : y, ox = p.up ? 2 * x + (z & 1) : x;
-    const size_t off = ((static_cast<size_t>(n) * oh + oy) * ow + ox) * p.channels + ch;
-    const float4 sc = *reinterpret_cast<const float4*>(p.scale + ch), sh = *reinterpret_cast<const float4*>(p.shift + ch);
-    float yv[4] = {fmaf(acc[0], sc.x, sh.x), fmaf(acc[1], sc.y, sh.y), fmaf(acc[2], sc.z, sh.z), fmaf(acc[3], sc.w, sh.w)};
-    if (p.has_res) {
-      for (int l = 0; l < p.nl; ++l) {
-        const uint2 r = *reinterpret_cast<const uint2*>(p.res + l * p.res_limb_stride + off);
-        if (p.nl == 2) {                          // PARITY: fp16 limbs
-          yv[0] += unpack_lo<true>(r.x); yv[1] += unpack_hi<true>(r.x); yv[2] += unpack_lo<true>(r.y); yv[3] += unpack_hi<true>(r.y);
-        } else {                                  // FAST: bf16
-          yv[0] += bf16_lo(r.x); yv[1] += bf16_hi(r.x); yv[2] += bf16_lo(r.y); yv[3] += bf16_hi(r.y);
-        }
-      }
-    }
-    if (p.relu) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) yv[i] = fmaxf(yv[i], 0.f);
-    }
-    if (p.nl == 2) {
-      uint2 o, lo;
-      o.x = pack2<true>(yv[0], yv[1]); o.y = pack2<true>(yv[2], yv[3]);
-      lo.x = pack2<true>(yv[0] - unpack_lo<true>(o.x), yv[1] - unpack_hi<true>(o.x));
-      lo.y = pack2<true>(yv[2] - unpack_lo<true>(o.y), yv[3] - unpack_hi<true>(o.y));
-      *reinterpret_cast<uint2*>(p.out + off) = o;
-      *reinterpret_cast<uint2*>(p.out + p.out_limb_stride + off) = lo;
-    } else {
-      uint2 o;
-      o.x = pack_bf16x2(yv[0], yv[1]); o.y = pack_bf16x2(yv[2], yv[3]);
-      *reinterpret_cast<uint2*>(p.out + off) = o;
-    }
+    finish4<NL>(p, pix, tc.nt * bn + g * 4, acc);
   }
 }
 

@@ -112,8 +112,7 @@ struct PlanLayer {
   int cluster = 1;        // CTAs per cluster sharing B stages by TMA multicast (patch mode only)
   bool split = false;     // split-K: conv kernel writes fp32 partials, splitk_reduce_kernel finishes
   int csplit = 0;         // split-K inside a cluster of this many CTAs (no finisher)
-  ReduceParams red;
-  int red_blocks = 0;
+  int red_blocks = 0;     // grid of splitk_reduce_kernel
 };
 
 struct IoKey {
@@ -451,9 +450,6 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 int nl_of(int mode) { return mode == LSPG_MODE_PARITY ? 2 : 1; }
 
-// conv_pair_kernel variant with stacked [B_hi; B_lo] operands (parity mode, N tile 64); see PairCfg
-bool pair_stacked(int bn, int NL) { return bn == 64 && NL == 2; }
-
 size_t tensor_bytes_one_limb(const TensorInfo& t, int B, int H, int W) {
   return static_cast<size_t>(B) * (H >> t.shift) * (W >> t.shift) * t.channels * 2;
 }
@@ -674,12 +670,6 @@ int make_weight_map_taps(lspg_ctx* h, CUtensorMap* m, const Layer& L, int bn, in
   return LSPG_OK;
 }
 
-int patch_tps(int bn, int NL, bool tail) {   // must mirror PatchCfg::kTPS
-  if (tail) return 9;
-  if (bn >= 128) return NL == 1 ? 2 : 1;
-  return NL == 1 ? 3 : 2;
-}
-
 uint32_t make_idesc(int bn, int m, bool f16) {
   // cute::UMMA::InstrDescriptor bit layout: c_format[4,6)=1 (F32), a_format[7,10) and b_format[10,13): 0 = F16, 1 = BF16,
   // a/b major [15],[16] = 0 (K-major), n_dim[17,23) = N>>3, m_dim[24,29) = M>>4
@@ -709,8 +699,6 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
     const Geo g = layer_geo(h, L, B, H, W);
     const int Hs = g.hs, Ws = g.ws;
     const int tw = g.tw, th = g.th, nb = g.nb;
-    // Measured on B200 (gpurun bringup2): the UMMA swizzle phase follows the absolute smem address, so a 128-byte-shifted
-    // start needs NO descriptor base offset (setting it corrupts the result).
     pl.patch = g.patch;
     int abox_w = tw, abox_h = th, abox_n = nb;
     if (pl.patch) {
@@ -728,7 +716,6 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
       for (int z = 0; z < L.n_phases; ++z)
         for (int t = 0; t < L.n_taps; ++t)
           p.tap_row[z][t] = static_cast<int16_t>((L.tap_dy[z][t] - p.patch_dy0[z]) * pw + (L.tap_dx[z][t] - p.patch_dx0[z]));
-      p.desc_base_offset = 0;
       if (pw * ph * 128 > kPatchSlot) return fail(LSPG_EINVAL, "patch %dx%d does not fit its smem slot", pw, ph);
       abox_w = pw; abox_h = ph; abox_n = 1;
     }
@@ -747,9 +734,7 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
     p.total_tiles = g.tiles_per_split * g.n_split;
     if (g.pair) {
       const int n_items = g.k_items * L.n_taps;                           // weight tiles per output tile
-      const int stage = (pair_stacked(g.bn, NL) ? 3 : NL) * (g.bn / 2) * 128;
-      const int cap = std::min(16, (kSmemBudget - 1024 - 5120 - 2 * NL * kPatchStride) / stage);
-      p.b_resident = (L.n_phases == 1 && g.n_tiles == 1 && n_items <= cap) ? 1 : 0;
+      p.b_resident = (L.n_phases == 1 && g.n_tiles == 1 && n_items <= pair_b_stages(g.bn, NL)) ? 1 : 0;
     }
     p.partial = reinterpret_cast<float*>(ws_scratch);
     // Split-K is two-pass: raw fp32 partials, then splitk_reduce_kernel.  (Measured on B200 in round 1: letting the
@@ -789,38 +774,28 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
     if (pl.patch) {
       pl.pair = g.pair;
       pl.cluster = g.csplit ? 1 : g.cluster;     // a cluster split launches CL = 1 code in clusters of csplit CTAs
-      if (pl.cluster == 1 && NL == 1 && !pl.pair) rc = make_weight_map_taps(h, &p.w, L, pl.bn, patch_tps(pl.bn, NL, L.kind == K_TAIL), NL);
+      if (pl.cluster == 1 && NL == 1 && !pl.pair) rc = make_weight_map_taps(h, &p.w, L, pl.bn, patch_taps_per_stage(pl.bn, NL, L.kind == K_TAIL), NL);
       else rc = make_weight_map_taps(h, &p.w, L, pl.bn / pl.cluster, 1, NL);      // per-tap boxes (row slice per CTA when multicasting)
       if (rc) return rc;
     } else {
       if ((rc = make_weight_map(h, &p.w, L, pl.bn, NL))) return rc;
     }
-    // ---- output / residual views
+    // ---- output / residual (the epilogue addresses both through plain pointers)
     if (L.kind != K_TAIL) {
-      const TensorInfo& t = h->tensors[L.out];
-      const int Ht = H >> t.shift, Wt = W >> t.shift;
-      void* tb = ws + P->tensor_off[L.out];
-      const size_t ls = P->tensor_limb_stride[L.out];
-      if (L.kind == K_UP) {
-        for (int q = 0; q < 4; ++q)
-          if ((rc = make_act_map(h, &p.out[q], tb, ls, NL, t.channels, B, Ht, Wt, true, q >> 1, q & 1, tw, th, nb))) return rc;
-      } else {
-        if ((rc = make_act_map(h, &p.out[0], tb, ls, NL, t.channels, B, Ht, Wt, false, 0, 0, tw, th, nb))) return rc;
-        for (int q = 1; q < 4; ++q) p.out[q] = p.out[0];
-      }
-      p.out_ptr = reinterpret_cast<__nv_bfloat16*>(tb);
-      p.out_limb_stride = static_cast<long long>(ls / 2);
-      p.out_channels = t.channels;
+      p.out_ptr = reinterpret_cast<__nv_bfloat16*>(ws + P->tensor_off[L.out]);
+      p.out_limb_stride = static_cast<long long>(P->tensor_limb_stride[L.out] / 2);
+      p.out_channels = h->tensors[L.out].channels;
       p.out_up = (L.kind == K_UP) ? 1 : 0;
       if (L.res >= 0) {
-        const TensorInfo& r = h->tensors[L.res];
         p.res_ptr = reinterpret_cast<const __nv_bfloat16*>(ws + P->tensor_off[L.res]);
         p.res_limb_stride = static_cast<long long>(P->tensor_limb_stride[L.res] / 2);
-        p.res_channels = r.channels;
+        p.res_channels = h->tensors[L.res].channels;
       }
-    } else {
-      for (int q = 0; q < 4; ++q) p.out[q] = p.a[0];
     }
+    // A split layer's output holds exactly its cout_pad channels, and its residual (only ever on stride-1 layers) has the
+    // output's grid and channel count: the split-K finishers rely on both, and build_network guarantees them.
+    if (g.n_split > 1 && (p.out_channels != L.cout_pad || (L.res >= 0 && (p.out_up || p.res_channels != p.out_channels))))
+      return fail(LSPG_EINVAL, "split-K layer %s: output/residual layout the split-K finishers do not support", L.conv_key.c_str());
     pl.grid = p.total_tiles < h->num_sms ? p.total_tiles : h->num_sms;
     if (pl.cluster > 1) pl.grid -= pl.grid % pl.cluster;
     {
@@ -834,19 +809,6 @@ int build_plan(lspg_ctx* h, Plan* P, int B, int H, int W, int mode, void* worksp
       }
     }
     if (pl.split) {
-      ReduceParams& r = pl.red;
-      memset(&r, 0, sizeof(r));
-      r.partial = p.partial; r.scale = p.scale; r.shift = L.d_shift;
-      r.out = reinterpret_cast<__nv_bfloat16*>(ws + P->tensor_off[L.out]);
-      r.out_limb_stride = static_cast<long long>(P->tensor_limb_stride[L.out] / 2);
-      if (L.res >= 0) {
-        r.res = reinterpret_cast<const __nv_bfloat16*>(ws + P->tensor_off[L.res]);
-        r.res_limb_stride = static_cast<long long>(P->tensor_limb_stride[L.res] / 2);
-      }
-      r.n_split = g.n_split; r.tiles_per_split = g.tiles_per_split; r.m_tiles = g.m_tiles; r.n_tiles = g.n_tiles;
-      r.n_phases = L.n_phases; r.tiles_x = p.tiles_x; r.tiles_y = p.tiles_y; r.tw_log2 = p.tw_log2; r.th_log2 = p.th_log2;
-      r.bn = g.bn; r.batch = B; r.hs = Hs; r.ws = Ws; r.up = (L.kind == K_UP) ? 1 : 0; r.channels = L.cout_pad;
-      r.relu = L.relu; r.has_res = L.res >= 0 ? 1 : 0; r.nl = NL;
       const long long work = static_cast<long long>(g.tiles_per_split) * kTileM * (g.bn / 4);   // one thread per pixel x 4 channels
       pl.red_blocks = static_cast<int>(std::min<long long>((work + 127) / 128, 8LL * h->num_sms));
     }
@@ -932,7 +894,7 @@ int launch_patch_cl(const ConvParams& p, int grid, int cluster, int device, cuda
 
 template <int BN, int NL>
 int launch_pair(const ConvParams& p, int grid, int device, cudaStream_t st) {
-  constexpr bool STK = (BN == 64 && NL == 2);          // must agree with pair_stacked()
+  constexpr bool STK = pair_stacked(BN, NL);
   using Cfg = PairCfg<BN, NL, STK>;
   static unsigned long long done = 0;
   int rc = ensure_smem(conv_pair_kernel<BN, NL, 8, STK>, Cfg::kSmemBytes, device, &done);
@@ -1020,7 +982,8 @@ int enqueue_forward(lspg_ctx* h, Plan* P, const IoKey& io, cudaStream_t st, bool
     if ((rc = launch_layer(pl, h->layers[i].kind, NL, h->device, st))) return rc;
     if (h->layers[i].kind == K_TAIL) h->tail_func = g_last_func;
     if (pl.split) {
-      CUDA_TRY(launch_pdl(splitk_reduce_kernel, dim3(pl.red_blocks), dim3(128), 0, st, pl.red));
+      if (NL == 1) CUDA_TRY(launch_pdl(splitk_reduce_kernel<1>, dim3(pl.red_blocks), dim3(128), 0, st, pl.prm, pl.bn));
+      else CUDA_TRY(launch_pdl(splitk_reduce_kernel<2>, dim3(pl.red_blocks), dim3(128), 0, st, pl.prm, pl.bn));
     }
     if (evs) CUDA_TRY(cudaEventRecord((*evs)[i + 2], st));
     if (debug_sync) {
